@@ -130,6 +130,8 @@ def main():
     ap.add_argument("--ref-md-steps", type=int, default=10)
     ap.add_argument("--dt", type=float, default=0.002)
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the last timed step, write DIR/positions.npy and DIR/velocities.npy (nm, nm/ps; float64)")
     args = ap.parse_args()
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -219,15 +221,24 @@ def main():
 
     # ---- end to end with HOST buffers: upload the state, run, read back positions + velocities + energy ----
     # --via plugin (default, single GPU): through the reference's public API -- Context.setPositions/setVelocities,
-    # LangevinIntegrator.step(md), Context.getState -- on the B200 Platform plugin (plugin/libOpenMMB200.so loaded into the
+    # LangevinIntegrator.step(md), Context.getState -- on the B200 Platform plugin (libOpenMMB200.so, plugin/, loaded into the
     # unmodified libOpenMM.so as its host application); --via cabi (and N > 1): the same calls on the bare C-ABI.
     x = eng.get_positions()
     v = eng.get_velocities()
+    if args.dump_outputs and rank == 0:
+        # every rank holds the same state; 48 bytes per atom, 47 MB for the largest workload (water1m)
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        np.save(os.path.join(args.dump_outputs, "positions.npy"), x)
+        np.save(os.path.join(args.dump_outputs, "velocities.npy"), v)
     via = args.via if world == 1 else "cabi"
     e2e_launches = 0
-    if via == "plugin":
+    e2e_sec = None
+    plugin_lib = os.path.join(ROOT, "oracle", "_ref", "plugins", "libOpenMMB200.so")
+    if via == "plugin" and not os.path.exists(plugin_lib):
+        pass                                  # the plugin needs the reference headers to build; reported as not measured below
+    elif via == "plugin":
         from oracle import omm                # the host application (reference libOpenMM.so + ctypes shim); compute is the plugin's
-        omm.load_plugin(os.path.join(ROOT, "plugin", "libOpenMMB200.so"))
+        omm.load_plugin(plugin_lib)
         sim = omm.Simulation(d, "B200", integrator=(systems.INT_LANGEVIN, 300.0, 1.0, args.dt), seed=7, constraint_tol=1e-5, pme=d.pme_parameters(),
                              props="DeviceIndex=%d" % local)
         assert sim.platform() == "B200"
@@ -260,7 +271,7 @@ def main():
         t = torch.tensor([e2e_sec])
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
         e2e_sec = float(t.item())
-    e2e_nsday = args.dt*1e-3*md*args.steps*86400/e2e_sec
+    e2e_nsday = args.dt*1e-3*md*args.steps*86400/e2e_sec if e2e_sec is not None else None
     nbytes = d.natoms*3*8
 
     if world > 1:
@@ -295,7 +306,8 @@ def main():
             "clocks": sampler.summary(),
             "e2e": {"value": e2e_nsday, "unit": "ns/day", "h2d_bytes_per_step": 2*nbytes, "d2h_bytes_per_step": 2*nbytes + 8,
                     "via": "OpenMM Platform plugin: Context.setPositions/setVelocities + LangevinIntegrator.step + Context.getState (libOpenMMB200.so)" if via == "plugin" else "C-ABI (b200md_set_positions/.../b200md_step)",
-                    "note": "per bench step: positions+velocities from host doubles, %d MD steps, positions+velocities back; final energy %.1f" % (md, e_final)},
+                    "note": ("per bench step: positions+velocities from host doubles, %d MD steps, positions+velocities back; final energy %.1f" % (md, e_final))
+                    if e2e_sec is not None else "not measured: the plugin library %s is not built" % os.path.relpath(plugin_lib, ROOT)},
             "gpu_launches": int(st1["kernel_launches"] - st0["kernel_launches"]),
             "roofline": {"kernel": "k_pair (direct-space 32x32 tile kernel)", "bound": "hbm", "achieved": achieved, "peak": peak, "unit": "GB/s", "frac": achieved/peak,
                          "traffic": traffic, "peak_source": peak_src, "algorithmic_bytes_per_launch": alg_bytes, "kernel_ms": pair_ms,

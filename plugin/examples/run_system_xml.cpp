@@ -7,7 +7,7 @@
 // openmm.app's ForceField.createSystem; tools/make_system_xml.py produces data-equivalent files from data/*.npz (built by
 // the reference's own forcefield.py, tools/make_benchmark_systems.py).
 //
-//   run_system_xml system.xml structure.pdb [--platform B200] [--plugin plugin/libOpenMMB200.so] [--steps 2000]
+//   run_system_xml system.xml structure.pdb [--platform B200] [--plugin oracle/_ref/plugins/libOpenMMB200.so] [--steps 2000]
 //                  [--dt 0.002] [--temperature 300] [--friction 1] [--device 0]
 // prints one JSON line: atoms, platform, ns/day, potential energy before / after.
 #include "openmm/Platform.h"
@@ -46,7 +46,7 @@ static std::vector<Vec3> readPdbPositions(const std::string& path) {
 
 int main(int argc, char** argv) {
     if (argc < 3) { fprintf(stderr, "usage: %s system.xml structure.pdb [--platform B200] [--plugin path] [--steps N] [--dt ps] [--temperature K] [--friction 1/ps] [--device i]\n", argv[0]); return 2; }
-    std::map<std::string, std::string> opt = {{"--platform", "B200"}, {"--plugin", "plugin/libOpenMMB200.so"}, {"--steps", "2000"}, {"--dt", "0.002"},
+    std::map<std::string, std::string> opt = {{"--platform", "B200"}, {"--plugin", "oracle/_ref/plugins/libOpenMMB200.so"}, {"--steps", "2000"}, {"--dt", "0.002"},
                                               {"--temperature", "300"}, {"--friction", "1"}, {"--device", "0"}};
     for (int i = 3; i + 1 < argc; i += 2) opt[argv[i]] = argv[i+1];
     try {

@@ -19,7 +19,7 @@ def _ngpu():
 def test_multi_gpu_engine_equals_single_gpu_engine(world, name):
     n = _ngpu()
     if n < world:
-        pytest.skip("needs %d GPUs on one box, this one has %d (run: gpurun --gpus %d -- python -m pytest tests/test_gpu_multi.py -m gpu)" % (world, n, world))
+        pytest.skip("needs %d GPUs on one box, this one has %d (run python -m pytest tests/test_gpu_multi.py -m gpu on a box with %d)" % (world, n, world))
     cmd = [sys.executable, "-m", "torch.distributed.run", "--nnodes=1", "--nproc-per-node", str(world), "--master-addr", "127.0.0.1",
            "--master-port", str(29400 + world), os.path.join(ROOT, "tests", "multi_rank_worker.py"), name, "40"]
     r = subprocess.run(cmd, capture_output=True, text=True, timeout=600, cwd=ROOT)

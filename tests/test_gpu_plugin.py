@@ -1,4 +1,4 @@
-"""GPU tests of the drop-in boundary proper: the B200 Platform plugin (plugin/libOpenMMB200.so) loaded into the
+"""GPU tests of the drop-in boundary proper: the B200 Platform plugin (libOpenMMB200.so, plugin/) loaded into the
 UNMODIFIED reference OpenMM (oracle/_ref/libOpenMM.so) through Platform::loadPluginLibrary, driven through the
 reference's public API (System / NonbondedForce / Context / LangevinIntegrator), compared with the Reference platform
 in the same process -- plus the reference's own test bodies (tests/Test<X>.h) built against the B200 platform."""
@@ -9,7 +9,7 @@ import pytest
 from conftest import relative_force_error, ROOT
 
 pytestmark = pytest.mark.gpu
-PLUGIN = os.path.join(ROOT, "plugin", "libOpenMMB200.so")
+PLUGIN = os.path.join(ROOT, "oracle", "_ref", "plugins", "libOpenMMB200.so")
 REFTESTS = os.path.join(ROOT, "oracle", "_ref", "tests")
 
 
@@ -17,7 +17,7 @@ REFTESTS = os.path.join(ROOT, "oracle", "_ref", "tests")
 def omm():
     from oracle import omm
     if not omm.available() or not os.path.exists(PLUGIN):
-        pytest.fail("oracle/_ref or the plugin is not built: run __graft_entry__.build() where /root/reference exists")
+        pytest.fail("oracle/_ref or the plugin is not built: run __graft_entry__.build() where the reference sources exist")
     omm.load_plugin(PLUGIN)
     assert "B200" in omm.platforms()
     return omm
@@ -106,7 +106,7 @@ def test_reference_own_test_bodies_pass_on_b200_platform(name):
     """tests/Test<X>.h of the reference compiled against our platform (plugin/tests/shim.cpp lists which functions)."""
     exe = os.path.join(REFTESTS, name)
     if not os.path.exists(exe):
-        pytest.fail("%s not built (make -C plugin reftests where /root/reference exists)" % exe)
+        pytest.fail("%s not built (make -C plugin reftests where the reference sources exist)" % exe)
     env = dict(os.environ, B200_PLUGIN=PLUGIN)
     for attempt in range(2):
         # the reference's statistical assertions (ASSERT_USUALLY_*: "This test is stochastic and may occasionally fail")
@@ -126,7 +126,7 @@ sys.path.insert(0, root)
 from openmm_b200 import systems
 from oracle import omm
 omm.load_plugin(os.path.join(root, "oracle", "_ref", "libOpenMMCPU.so"))
-plug = os.path.join(root, "plugin", "libOpenMMB200Pme.so")
+plug = os.path.join(root, "oracle", "_ref", "plugins", "libOpenMMB200Pme.so")
 omm.load_plugin(plug)                         # registers "CalcPmeReciprocalForce" on the Reference and CPU platforms
 count = ctypes.CDLL(plug).b200pme_exec_count
 count.restype = ctypes.c_long
@@ -148,7 +148,7 @@ print("RESULT", n1 - n0, err.max(), abs(ec - er)/abs(er), errt.max(), abs(et - e
 
 @pytest.mark.gpu
 def test_standalone_pme_kernel_serves_the_reference_cpu_platform():
-    """SURVEY.md 8f rank 3: plugin/libOpenMMB200Pme.so registers a "CalcPmeReciprocalForce" kernel (kernels.h:1493-1557, the
+    """SURVEY.md 8f rank 3: libOpenMMB200Pme.so (plugin/B200PmePlugin.cpp) registers a "CalcPmeReciprocalForce" kernel (kernels.h:1493-1557, the
     plugins/cpupme pattern).  The UNMODIFIED reference CPU platform then routes reciprocal space through the bespoke
     spread / FFT / convolution / gather (CpuKernels.cpp:620-690) and must still agree with the Reference platform."""
     import sys
@@ -173,7 +173,7 @@ def test_cpp_host_application_loads_system_xml_and_pdb(omm, tmp_path):
     import sys
     exe = os.path.join(REFTESTS, "run_system_xml")
     if not os.path.exists(exe):
-        pytest.fail("run_system_xml not built (make -C plugin reftests where /root/reference exists)")
+        pytest.fail("run_system_xml not built (make -C plugin reftests where the reference sources exist)")
     base = str(tmp_path/"dhfr")
     r = subprocess.run([sys.executable, os.path.join(ROOT, "tools", "make_system_xml.py"), "dhfr", base], capture_output=True, text=True, timeout=300)
     assert r.returncode == 0, r.stdout + r.stderr
